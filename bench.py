@@ -251,7 +251,7 @@ def parity_record(name, dev):
     from tests.helpers import CodebookAux, build_ar, noise_tensor
     gold = os.path.join(ROOT, "tests", "golden")
     g, fixture = None, None
-    for fixture in ("ar.pt", "ar2.pt"):
+    for fixture in ("ar.pt", "ar2.pt", "ar3.pt"):
         g = torch.load(os.path.join(gold, fixture), weights_only=False)["ar"].get(name)
         if g is not None:
             break
@@ -299,6 +299,29 @@ def parity_record(name, dev):
             "free_running": free}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, codes, pix, rank, world):
+    """What a caller of the timed path receives -- the [B,H,W,D] code maps and the [B,3,R,R] pixels in [0,1] -- as float32
+    .npy files, so that two builds can be compared output for output on identical seeded inputs.  All ranks together stay
+    within DUMP_BYTES: when the pixels do not fit, a fixed seeded subset of the images is written, with their batch indices
+    in pixels_index.npy."""
+    import numpy as np
+    sfx = "_rank%d" % rank if world > 1 else ""
+    codes = codes.float().cpu().numpy()
+    pix = pix.float().cpu().numpy()
+    per_image = pix[0].nbytes
+    keep = max(1, min(len(pix), (DUMP_BYTES // max(world, 1) - codes.nbytes - 8 * len(pix)) // per_image))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "codes%s.npy" % sfx), codes)
+    if keep < len(pix):
+        idx = np.sort(np.random.default_rng(0).choice(len(pix), keep, replace=False))
+        pix = pix[idx]
+        np.save(os.path.join(out_dir, "pixels_index%s.npy" % sfx), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "pixels%s.npy" % sfx), pix)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -313,7 +336,12 @@ def main():
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the exact_tier and strong records")
     ap.add_argument("--cpu-budget", type=float, default=25.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the codes and pixels of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; --impl reference times a bounded sample of the CPU path")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -390,6 +418,7 @@ def main():
             if e2e:
                 io["pix_h"].copy_(pix, non_blocking=True)
             ev[i][2].record()
+            io["last"] = (codes, pix)
         t1.record()
         barrier()
         total = t0.elapsed_time(t1)
@@ -409,6 +438,8 @@ def main():
     total, ar_ms, dec_ms = timed(io, False, args.steps)
     clock_summary = clocks.summary() if rank == 0 else None
     launches = N.launch_count["total"] - launches0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *io["last"], rank, world)
     timed(io, True, 1)
     e_total, e_ar, e_dec = timed(io, True, args.steps)
 

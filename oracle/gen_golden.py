@@ -23,7 +23,7 @@ from oracle import synth                    # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden")
 
-from oracle.zoo import AR_ZOO, VAE_ZOO      # noqa: E402
+from oracle.zoo import AR2_FILES, AR_ZOO, VAE_ZOO      # noqa: E402
 
 
 def ar_cfg(name):
@@ -139,14 +139,30 @@ def gen_sampler(ns, out):
 
 
 def gen_ar2(ns, out):
-    """second batch of AR fixtures (tests/golden/ar2.pt): the text-conditioned BASELINE shapes (configs 4 / 5) -- 32-token prefix
-    prefill, the synthetic 16x16x4 grid, the 3.9B widths.  Same protocol as gen_ar."""
+    """second batch of AR fixtures (tests/golden/ar2.pt, ar3.pt): the text-conditioned BASELINE shapes (configs 4 / 5) -- 32-token
+    prefix prefill, the synthetic 16x16x4 grid, the 3.9B widths.  Same protocol as gen_ar."""
     plan = [
         ("cc3m654m", 2, [dict(top_k=1), dict(top_k=1024, top_p=0.95)], [0, 1, 4, 255]),
         ("cc3m654m_16", 2, [dict(top_k=1024, top_p=0.95)], [0, 5, 1023]),
         ("t2i3900m", 2, [dict(top_k=1024, top_p=0.95)], [0, 1, 7, 255]),
     ]
     out["ar"] = _gen_ar_plan(ns, plan, keep_logits_of=lambda si: True)
+
+
+def save_ar2(res):
+    """writes AR2_FILES; logits that two runs of a model share bit for bit (the runs have not diverged yet: step 0) are stored
+    once, as one tensor referenced from both runs"""
+    for g in res.values():
+        kept = []
+        for run in g["runs"]:
+            for step, lg in (run["logits"] or {}).items():
+                same = next((t for t in kept if torch.equal(t, lg)), None)
+                if same is None:
+                    kept.append(lg)
+                else:
+                    run["logits"][step] = same
+    for fixture, names in AR2_FILES.items():
+        torch.save({"ar": {n: res[n] for n in names}}, os.path.join(GOLD, fixture + ".pt"))
 
 
 def gen_ar(ns, out):
@@ -248,21 +264,117 @@ def gen_layouts(ns):
         json.dump(lay, f)
 
 
+def gen_seeded_init(ns):
+    """the reference's default initialisation after torch.manual_seed(0) (tests/test_host_cpu.py)"""
+    E, nh, nb, nhl, V, bs, vc, cl = AR_ZOO["tiny"]
+    torch.manual_seed(0)
+    ar = ns.RQTransformer(R.transformer_cfg(E, nh, nb, nhl, V, block_size=bs, vocab_cond=vc, cond_len=cl))
+    torch.manual_seed(0)
+    vae = ns.RQVAE(**R.vae_kwargs(**VAE_ZOO["tiny"]))
+    with open(os.path.join(GOLD, "seeded_init.json"), "w") as f:
+        json.dump({"ar/tiny": synth.tensor_digests(ar.state_dict()), "vae/tiny": synth.tensor_digests(vae.state_dict())}, f)
+
+
+SCRIPTS = {"measure_throughput": os.path.join("measure_throughput", "__main__.py"),
+           "main_sampling_fid": "main_sampling_fid.py",
+           "compute_metrics": "compute_metrics.py"}          # imported by main_sampling_fid
+
+
+def script_imports(path):
+    """[[module, name or None], ...]: what a script imports from the modules this repository provides (``rqvae`` and the
+    ``compat`` omegaconf / easydict stand-ins), read from its source with ast"""
+    import ast
+    with open(path) as f:
+        tree = ast.parse(f.read())
+    ours = ("rqvae", "omegaconf", "easydict")
+    found = []
+    for node in ast.walk(tree):
+        if isinstance(node, ast.Import):
+            found += [[a.name, None] for a in node.names if a.name.split(".")[0] in ours]
+        elif isinstance(node, ast.ImportFrom) and node.level == 0 and node.module.split(".")[0] in ours:
+            found += [[node.module, a.name] for a in node.names]
+    return found
+
+
+def gen_scripts(ns):
+    """what the reference's own scripts take from this repository's ``rqvae`` package (tests/test_reference_scripts_cpu.py):
+    every name they import from it; measure_throughput's Experiment fields and the arch configs it passes to
+    augment_arch_defaults for `f=32 d=4 c=2048 model=small` and `f=32 d=4 c=16384 model=huge`; and the configs
+    main_sampling_fid.load_model() reads back from a checkpoint directory written with the tiny test configs (that function
+    calls this package's load_config / augment_arch_defaults, so those are a snapshot of this package's output)."""
+    import dataclasses
+    import importlib.util
+    import tempfile
+    import yaml
+    pkg = os.path.join(ROOT, "rq-vae-transformer_b200")
+    added = [pkg, os.path.join(pkg, "compat"), R.REFERENCE_ROOT]     # ours shadows the reference's `rqvae`
+    sys.path.insert(0, added[0])
+    sys.path.extend(added[1:])
+    out = {"imports": {k: script_imports(os.path.join(R.REFERENCE_ROOT, rel)) for k, rel in SCRIPTS.items()}}
+    try:
+        def load(name, rel):
+            spec = importlib.util.spec_from_file_location(name, os.path.join(R.REFERENCE_ROOT, rel))
+            mod = importlib.util.module_from_spec(spec)
+            spec.loader.exec_module(mod)
+            return mod
+
+        mt = load("ref_measure_throughput", SCRIPTS["measure_throughput"])
+        out["measure_throughput"] = {"experiment_fields": [[f.name, f.type if isinstance(f.type, str) else f.type.__name__, f.default]
+                                                           for f in dataclasses.fields(mt.Experiment)],
+                                     "create_model": []}
+        augment = mt.augment_arch_defaults
+        for args in (("f32", "small", 4, 2048), ("f32", "huge", 4, 16384)):
+            seen = []
+            mt.augment_arch_defaults = lambda c: (seen.append(c.to_dict()), augment(c))[1]
+            with torch.device("meta"):
+                mt.create_model(*args)
+            mt.augment_arch_defaults = augment
+            out["measure_throughput"]["create_model"].append({"args": list(args), "rqvae": seen[0], "rqtransformer": seen[1]})
+
+        msf = load("ref_main_sampling_fid", SCRIPTS["main_sampling_fid"])
+        from tests.helpers import ar_config, vae_config
+        from rqvae.models import create_model
+        out["main_sampling_fid"] = {}
+        with tempfile.TemporaryDirectory() as tmp:
+            for name, cfg in (("ar", ar_config("tiny")), ("vae", vae_config("tiny"))):
+                os.makedirs(os.path.join(tmp, name))
+                model, _ = create_model(cfg)
+                torch.save({"state_dict": model.state_dict(), "state_dict_ema": model.state_dict()}, os.path.join(tmp, name, "model.pt"))
+                written = {"arch": cfg.to_dict(), "dataset": {"type": "imagenet"},
+                           "sampling": {"temp": 1.0, "top_k": [1024], "top_p": [0.95]}}
+                with open(os.path.join(tmp, name, "config.yaml"), "w") as f:
+                    yaml.safe_dump(written, f)
+                _, config = msf.load_model(os.path.join(tmp, name, "model.pt"), ema=(name == "ar"))
+                out["main_sampling_fid"][name] = {"config_yaml": written, "loaded": config.to_dict()}
+    finally:
+        for p in added:
+            sys.path.remove(p)
+    with open(os.path.join(GOLD, "reference_scripts.json"), "w") as f:
+        json.dump(out, f, indent=1)
+
+
 def main():
     torch.set_grad_enabled(False)
     os.makedirs(GOLD, exist_ok=True)
     ns = R.load_reference()
     check_multinomial_identity()
-    which = sys.argv[1:] or ["rq", "sampler", "ar", "vae", "ar2", "layouts"]
+    which = sys.argv[1:] or ["rq", "sampler", "ar", "vae", "ar2", "layouts", "init", "scripts"]
     for part, fn in (("rq", gen_rq), ("sampler", gen_sampler), ("ar", gen_ar), ("vae", gen_vae), ("ar2", gen_ar2)):
         if part in which:
             out = {}
             t0 = time.time()
             fn(ns, out)
-            torch.save(out, os.path.join(GOLD, part + ".pt"))
+            if part == "ar2":
+                save_ar2(out["ar"])
+            else:
+                torch.save(out, os.path.join(GOLD, part + ".pt"))
             print("%s done in %.1fs" % (part, time.time() - t0), flush=True)
     if "layouts" in which:
         gen_layouts(ns)
+    if "init" in which:
+        gen_seeded_init(ns)
+    if "scripts" in which:
+        gen_scripts(ns)
     meta = dict(torch=torch.__version__, threads=torch.get_num_threads(), reference="kakaobrain/rq-vae-transformer@341395e")
     with open(os.path.join(GOLD, "META.json"), "w") as f:
         json.dump(meta, f)

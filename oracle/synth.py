@@ -8,6 +8,7 @@ oracle and the CUDA engine (on the GPU box, where the reference is absent) all g
 defaults (Linear/Conv: U(+-1/sqrt(fan_in)); Embedding: N(0,1); pos_emb: N(0,0.02), transformers.py:79-81) except
 that norm layers get a non-trivial affine (1+0.1 N, 0.1 N) so that the affine path is actually exercised.
 """
+import hashlib
 import math
 
 import torch
@@ -69,6 +70,12 @@ def re_norm(k):
 
 def shapes_of(state_dict):
     return {k: tuple(v.shape) for k, v in state_dict.items()}
+
+
+def tensor_digests(state_dict):
+    """{key: [shape, sha256 of the raw bytes]} -- pins a state dict bit for bit without storing its values"""
+    return {k: [list(v.shape), hashlib.sha256(v.detach().contiguous().cpu().numpy().tobytes()).hexdigest()]
+            for k, v in state_dict.items()}
 
 
 def randn_seeded(shape, seed, scale=1.0):

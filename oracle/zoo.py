@@ -20,6 +20,14 @@ VAE_ZOO = {
     "imagenet": dict(K=16384, attn_resolutions=(8,)),             # configs/imagenet256/stage1/in256-rqvae-8x8x4.yaml:12,30
 }
 
+# golden files of the reference's AR trajectories beyond tests/golden/ar.pt, split so that every file stays under 1 MB
+AR2_FILES = {"ar2": ("cc3m654m",), "ar3": ("cc3m654m_16", "t2i3900m")}
+
+
+def ar_fixture(name):
+    """the tests/golden/<fixture>.pt holding the reference's AR trajectories of model `name`"""
+    return next((f for f, names in AR2_FILES.items() if name in names), "ar")
+
 
 def vae_ddconfig(K, code_shape=(8, 8, 4), embed_dim=256, ch=128, ch_mult=(1, 1, 2, 2, 4, 4), attn_resolutions=(8,),
                  resolution=256, z_channels=256, num_res_blocks=2):

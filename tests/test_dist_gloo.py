@@ -3,6 +3,7 @@ all_gather of code maps (SURVEY.md 8e).  No kernels run here."""
 import os
 import socket
 import sys
+from unittest import mock
 
 import torch
 import torch.distributed as dist
@@ -59,8 +60,10 @@ def test_two_rank_gloo_sharding_and_gather():
     q = ctx.Queue()
     port = _free_port()
     procs = [ctx.Process(target=_worker, args=(r, 2, port, q)) for r in range(2)]
-    for p in procs:
-        p.start()
+    # CPU-only ranks: with a GPU visible, rank r would claim cuda:r, which a one-GPU machine does not have
+    with mock.patch.dict(os.environ, {"CUDA_VISIBLE_DEVICES": ""}):
+        for p in procs:
+            p.start()
     for p in procs:
         p.join(120)
         assert p.exitcode == 0

@@ -10,7 +10,7 @@ import pytest
 import torch
 
 from oracle import synth
-from oracle.zoo import AR_ZOO
+from oracle.zoo import AR_ZOO, ar_fixture
 from tests.helpers import CodebookAux, build_ar, noise_tensor
 
 pytestmark = pytest.mark.gpu
@@ -19,7 +19,7 @@ DEV = "cuda"
 
 
 def _case(name, golden, layouts):
-    g = golden("ar2" if name in ("cc3m654m", "cc3m654m_16", "t2i3900m") else "ar")["ar"][name]
+    g = golden(ar_fixture(name))["ar"][name]
     E, nh, nb_, nhl, V, bs, vc, cl = AR_ZOO[name]
     model, sd = build_ar(name, layouts, g["weight_seed"])
     cb = synth.randn_seeded((V, 256), g["codebook_seed"]).to(DEV)
